@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline measurement of the AdaIN-VC hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--c-in 80] [--batch 256]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--c-in 80] [--batch 256] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 A "step" is one full Solver train step (forward + backward + grad-norm clip + Adam/amsgrad)
@@ -16,6 +16,18 @@ weak scaling, config 4, for N > 1).  Prints ONE JSON line (rank 0).
             timed alone with CUDA events on rotating >L2 buffers.
   cpu_baseline / --impl reference: the CPU oracle port of the reference path
             (oracle/ae_oracle.py, torch CPU fp32, all host threads) on a bounded sample.
+
+--dump-outputs DIR: after the timed steps, the parameters and the optimizer state are put back to what they
+were before the first step, and one more step runs through the timed path (the captured graph, called through
+Solver.ae_step on the first host batch).  That step's losses and the gradient it computed are written as
+DIR/<name>.npy.  Weights, batch and noise are seeded, so this step has the same inputs on every run (for a
+given --c-in, --batch and number of GPUs), and its outputs differ between runs only by the rounding of the
+reductions that add with atomics (bias and weight gradients, loss sums).  On a B200 (1000 W power limit),
+runs at --steps 20 and 3 agreed to 1.1e-7 relative L2 on the gradient and 4e-7 relative on the losses.
+The chained timed steps are not what is dumped: every Adam step carries that rounding into the next, and a
+weight whose gradient is analytically zero (a bias in front of an InstanceNorm) moves by +-lr in the direction
+of its rounding noise, so after the timed steps two runs of one build are far apart.  For the same reason the
+updated parameters are not dumped.
 """
 from __future__ import annotations
 
@@ -62,7 +74,13 @@ def parse():
                          "per pinned host batch (the reference's blocking call)")
     ap.add_argument("--workload", default="train", choices=["train", "inference"],
                     help="train: BASELINE config 3/4 (default, the headline metric); inference: config 5, 64 (src,tgt) pairs of 80x512")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, run one step from the initial parameters and optimizer state through the timed path "
+                         "and write its losses and gradient as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl, args.workload) != ("b200", "train"):
+        ap.error("--dump-outputs writes the outputs of the training step of --impl b200 --workload train")
+    return args
 
 
 def config_for(c_in, batch):
@@ -315,12 +333,16 @@ def run_b200(args):
                                   load_opt=False, store_model_path=None, load_model_path=None, summary_steps=10 ** 9,
                                   save_steps=10 ** 9, tag="bench", iters=0)
     import contextlib, io
+    torch.manual_seed(0)   # the initial weights and the reparameterisation noise: the same on every run
     with contextlib.redirect_stdout(io.StringIO()):
         solver = Solver(cfg, sargs)
     tr = solver.trainer
     B, K, W = args.batch, args.steps, max(args.warmup, 3)
     host_batches = solver.train_loader.batches          # pinned host N(0,1) batches (seed 1+rank)
     x_dev = host_batches[0].to(dev)
+    opt = solver.opt
+    step_state = [opt.flat_p, opt.flat_m, opt.flat_v, opt.flat_vmax, opt.step_dev]   # what a step reads and updates
+    initial_state = [t.clone() for t in step_state] if args.dump_outputs else None
 
     def barrier():
         if world > 1:
@@ -375,6 +397,14 @@ def run_b200(args):
     ms, ms_e2e = sorted(win)[len(win) // 2], sorted(win_e2e)[len(win_e2e) // 2]
     finite = all(map(lambda v: v == v and abs(v) != float("inf"), meta.values()))
     precision = tr.eng.precision
+    if args.dump_outputs:   # every rank takes the step (it all-reduces); rank 0 writes it
+        for t, t0 in zip(step_state, initial_state):
+            t.copy_(t0)
+        tr.eng.pack_weights(tr.P, need_dgrad=True)
+        torch.manual_seed(0)   # its noise, whatever --steps and --warmup ran before
+        losses = solver.ae_step(host_batches[0], 1.0)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, losses, opt.flat_g)
 
     if rank == 0:
         value = B * world * K / (ms * 1e-3)
@@ -415,6 +445,24 @@ def run_b200(args):
         line["cpu_baseline"] = {"value": rate, "unit": UNIT, "cores": cores, "kind": "port",
                                 "sample": f"3 steps of batch {B} after 1 warm-up (oracle port of the reference Solver.ae_step, torch CPU fp32, best of a thread sweep: {cores} of {os.cpu_count()} threads), {spt:.2f} s/step"}
     print(json.dumps(line), flush=True)
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, losses, flat_g):
+    """What the dumped step computed, as out_dir/<name>.npy: the losses Solver.ae_step returns (float64
+    scalars) and the step's gradient (float32, flattened in model.parameters() order).  Gradient elements
+    beyond the dump's 64 MB are replaced by a fixed, seeded sample of them, in index order."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, value in losses.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.float64(value))
+    g = flat_g.detach().cpu()
+    keep = (DUMP_BYTES - 4096) // 4
+    if g.numel() > keep:
+        g = g[torch.randperm(g.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values]
+    np.save(os.path.join(out_dir, "gradients.npy"), g.numpy())
 
 
 def _quick_train_rate(c_in, batch, dev, steps, precision=None):

@@ -129,6 +129,19 @@ def make_infer_fixture(ref_model, c_in, batch, T, T_cond, name):
     print(name, tuple(dec.shape))
 
 
+def make_reference_forward_fixture(ref_model, name):
+    """One forward pass of the reference AE, recorded with the seeds of train_c80_b1.pt's first step, so that
+    the suite can check that fixture and the oracle against the reference without the reference itself."""
+    import oracle.ae_oracle as orc
+    config = orc.default_config(80)
+    x = randn((1, 80, 128), seed=1)
+    with torch.no_grad():
+        _, mu, ls, emb, dec = run_ae(ref_model, config, orc.init_state(config, seed=0), x, eps_seed=100)
+    torch.save({"x": x, "eps_seed": 100, "mu": mu, "log_sigma": ls, "emb": emb, "dec": dec},
+               os.path.join(ROOT, "tests", "golden", name))
+    print(name, tuple(dec.shape))
+
+
 def make_helper_fixture(ref_model, name):
     """Known answers for the small helpers of model.py:21-32, 52-63, 77-83."""
     x = randn((2, 8, 11), seed=5)
@@ -165,6 +178,7 @@ def main():
     make_train_fixture(ref_model, 512, 2, 128, 1, "train_c512_b2.pt")    # shipped config.yaml
     make_infer_fixture(ref_model, 80, 2, 301, 173, "infer_c80.pt")       # odd lengths, T_cond != T
     make_infer_fixture(ref_model, 80, 1, 512, 512, "infer_c80_t512.pt")  # BASELINE config 5 shape
+    make_reference_forward_fixture(ref_model, "reference_fwd_c80_b1.pt")
 
 
 if __name__ == "__main__":

@@ -87,6 +87,33 @@ def test_bench_reference_arm_schema():
     assert d["config"] == want      # the very dict the product arm prints (arm-specific facts live under "run")
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: one float64 .npy per loss, the gradient in float32, and a fixed sample of
+    the gradient when it exceeds the dump's size limit."""
+    import importlib.util, os, sys
+    import numpy as np
+    from conftest import ROOT
+    spec = importlib.util.spec_from_file_location("avc_bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    g = torch.randn(1000)
+    losses = {"loss_rec": 1.5, "loss_kl": 0.25, "grad_norm": 3.0}
+    bench.dump_outputs(str(tmp_path / "a"), losses, g)
+    for k, v in losses.items():
+        a = np.load(tmp_path / "a" / f"{k}.npy")
+        assert a.dtype == np.float64 and float(a) == v
+    a = np.load(tmp_path / "a" / "gradients.npy")
+    assert a.dtype == np.float32 and np.array_equal(a, g.numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096 + 4 * 100)
+    bench.dump_outputs(str(tmp_path / "b"), losses, g)
+    bench.dump_outputs(str(tmp_path / "c"), losses, g)
+    b, c = np.load(tmp_path / "b" / "gradients.npy"), np.load(tmp_path / "c" / "gradients.npy")
+    assert b.shape == (100,) and np.array_equal(b, c) and np.isin(b, a).all()
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--impl", "reference", "--dump-outputs", str(tmp_path)])
+    with pytest.raises(SystemExit):
+        bench.parse()
+
+
 def test_cli_flags_match_reference_names():
     """main.py keeps the reference's flag names (main.py:9-22 of the reference)."""
     import importlib.util, os

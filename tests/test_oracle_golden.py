@@ -89,19 +89,21 @@ def test_inference(golden_dir, name):
     assert rel(emb, fx["emb"]) < 2e-4
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree only exists in the authoring container")
 def test_live_reference_matches_fixture(golden_dir):
-    """Re-run the unmodified reference and compare with the committed fixture (guards the
-    fixture generator itself)."""
-    from oracle.make_golden import import_reference
-    ref_model = import_reference()
+    """A forward pass of the unmodified reference, recorded by oracle/make_golden.py, against the
+    training fixture made from the same seeds (guards the fixture generator itself) and against
+    the oracle fed the noise the reference draws after seeding torch's generator."""
+    from oracle.make_golden import reference_eps
+    ref = load(golden_dir, "reference_fwd_c80_b1.pt")
     fx = load(golden_dir, "train_c80_b1.pt")
+    assert torch.equal(ref["x"], fx["x"])
+    assert rel(ref["dec"], fx["steps"][0]["dec"]) < 1e-5
     cfg = orc.default_config(80)
-    ae = ref_model.AE(cfg)
-    ae.load_state_dict(orc.init_state(cfg, seed=0), strict=True)
-    torch.manual_seed(100)
-    mu, ls, emb, dec = ae(fx["x"])
-    assert rel(dec, fx["steps"][0]["dec"]) < 1e-5
+    eps = reference_eps(ref["log_sigma"].shape, ref["eps_seed"])
+    with torch.no_grad():
+        mu, ls, emb, dec = orc.ae_forward(orc.init_state(cfg, seed=0), cfg, ref["x"], eps)
+    for k, v in (("mu", mu), ("log_sigma", ls), ("emb", emb), ("dec", dec)):
+        assert rel(v, ref[k]) < 2e-4, (k, rel(v, ref[k]))
 
 
 def test_torch_optim_step_agrees_with_restated_adam(golden_dir):
