@@ -102,6 +102,11 @@ class DenseStackDesc(C.Structure):
     ]
 
 
+class SnItem(C.Structure):
+    _fields_ = [("w_orig", _fp), ("w_sn", _fp), ("u", _fp), ("v", _fp), ("sigma", _fp), ("grad", _fp),
+                ("rows", C.c_int32), ("cols", C.c_int32)]
+
+
 LINEAR_BATCH_MAX = 16
 
 
@@ -158,6 +163,8 @@ PROTOTYPES = {
     "avc_sqnorm": (_i, [_p, _i64, _p, _p, _p]),
     "avc_adam_step": (_i, [_p, _p, _p, _p, _p, _i64, _p, _p, _p, _p]),
     "avc_fill_zero": (_i, [_p, _i64, _p]),
+    "avc_spectral_norm_fwd": (_i, [_p, _i, _i, _p]),
+    "avc_spectral_norm_bwd": (_i, [_p, _i, _p]),
     "avc_tc_probe_gemm": (_i, [_p, _i, _p, _i, C.POINTER(C.c_uint32), _i, _i, _i, _i, _i, _p, _p, _p]),
     "avc_tc_probe_set_ld_shift": (None, [_i]),
     "avc_probe_store": (_i, [_p, C.c_longlong, _i, _i, _p, _p]),

@@ -81,8 +81,8 @@ class Engine:
         for c in (se, ce):
             if c.get("act", "relu") != "relu" or c.get("dropout_rate", 0) != 0:
                 raise L.AvcError("only act='relu', dropout_rate=0 (the reference config.yaml) are implemented")
-        if de.get("act", "relu") != "relu" or de.get("dropout_rate", 0) != 0 or de.get("sn", False):
-            raise L.AvcError("Decoder: only act='relu', dropout_rate=0, sn=False are implemented")
+        if de.get("act", "relu") != "relu" or de.get("dropout_rate", 0) != 0:
+            raise L.AvcError("Decoder: only act='relu', dropout_rate=0 are implemented")
         for up in de["upsample"]:
             if up not in (1, 2):
                 raise L.AvcError("Decoder.upsample entries must be 1 or 2")

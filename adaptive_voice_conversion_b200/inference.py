@@ -85,8 +85,8 @@ class Inferencer(object):
 
     def _param_version(self):
         # in-place updates (optimizer steps, load_state_dict) bump a tensor's version counter: a captured graph reads
-        # the weight packs of the version it was captured with
-        return sum(int(p._version) for p in self.model.parameters())
+        # the weight packs of the version it was captured with (and, with sn, the u / v buffers sigma is computed from)
+        return sum(int(t._version) for t in list(self.model.parameters()) + list(self.model.buffers()))
 
     @torch.no_grad()
     def inference_ragged(self, xs, x_conds):

@@ -79,17 +79,21 @@ class ContentEncoder(_ParamStack):
 
 
 class Decoder(_ParamStack):
-    """Parameters of the reference Decoder (model.py:325-345)."""
+    """Parameters of the reference Decoder (model.py:325-345).  With ``sn`` every layer is registered through
+    ``torch.nn.utils.spectral_norm`` like the reference's: parameters ``bias``, ``weight_orig`` and buffers
+    ``weight_u``, ``weight_v`` per layer, and the ``spectral_norm`` state_dict metadata.  torch's forward hook
+    never runs (the containers are not called) and the plain ``weight`` attribute it leaves behind is never
+    read: the effective weights W/sigma are computed by ``AE`` (csrc/spectral_norm.cu)."""
 
     def __init__(self, c_in, c_cond, c_h, c_out, kernel_size, n_conv_blocks, upsample, act, sn, dropout_rate):
         super().__init__()
-        if sn:
-            raise L.AvcError("spectral norm (sn=True) is not implemented; the reference config uses sn: False")
-        self.in_conv_layer = nn.Conv1d(c_in, c_h, kernel_size=1)
-        self._convs("first_conv_layers", [(c_h, c_h, kernel_size, 1)] * n_conv_blocks)
-        self._convs("second_conv_layers", [(c_h, c_h * up, kernel_size, 1) for _, up in zip(range(n_conv_blocks), upsample)])
-        self._linears("conv_affine_layers", [(c_cond, c_h * 2)] * (2 * n_conv_blocks))
-        self.out_conv_layer = nn.Conv1d(c_h, c_out, kernel_size=1)
+        f = nn.utils.spectral_norm if sn else (lambda m: m)
+        self.in_conv_layer = f(nn.Conv1d(c_in, c_h, kernel_size=1))
+        self.first_conv_layers = nn.ModuleList([f(nn.Conv1d(c_h, c_h, kernel_size=kernel_size)) for _ in range(n_conv_blocks)])
+        self.second_conv_layers = nn.ModuleList([f(nn.Conv1d(c_h, c_h * up, kernel_size=kernel_size))
+                                                 for _, up in zip(range(n_conv_blocks), upsample)])
+        self.conv_affine_layers = nn.ModuleList([f(nn.Linear(c_cond, c_h * 2)) for _ in range(2 * n_conv_blocks)])
+        self.out_conv_layer = f(nn.Conv1d(c_h, c_out, kernel_size=1))
 
 
 def _check_input(x: torch.Tensor, what: str) -> torch.Tensor:
@@ -109,6 +113,9 @@ class _StackFn(torch.autograd.Function):
         names = model._names_by_prefix[prefix]
         P = dict(zip(names, params))
         eng = model.engine(params[0].device)
+        if prefix == "decoder." and model.sn:
+            model.spectral_norm_fwd(params[0].device, update=model.training)
+            P, _ = model.sn_views(P)
         eng.pack_weights(P, need_dgrad=train, prefixes=(prefix,))
         ctx.model, ctx.prefix, ctx.P, ctx.train = model, prefix, P, train
         return eng, P
@@ -181,12 +188,18 @@ class _DecoderFn(_StackFn):
 
     @staticmethod
     def backward(ctx, ddec):
-        eng = ctx.model.engine(ddec.device)
+        model = ctx.model
+        eng = model.engine(ddec.device)
         G, names = _StackFn._grads(ctx, eng)
         B, Cc, T = ddec.shape
         ddec4 = A4.empty(B, Cc, T, ddec.device)
         eng.pack_a4(ddec.contiguous(), ddec4)
-        dz4, demb = eng.decoder_bwd(ctx.P, G, ctx.saved, ddec4)
+        if model.sn:
+            _, Gk = model.sn_views(ctx.P, G)
+            dz4, demb = eng.decoder_bwd(ctx.P, Gk, ctx.saved, ddec4)
+            model.spectral_norm_bwd(Gk)
+        else:
+            dz4, demb = eng.decoder_bwd(ctx.P, G, ctx.saved, ddec4)
         dmu4, dls4 = eng.reparam_bwd(dz4, ctx.ls4, ctx.eps, None, None)
         dmu, dls = eng.unpack_a4(dmu4), eng.unpack_a4(dls4)
         ctx.saved = None
@@ -202,6 +215,8 @@ class AE(nn.Module):
         self.speaker_encoder = SpeakerEncoder(**config["SpeakerEncoder"])
         self.content_encoder = ContentEncoder(**config["ContentEncoder"])
         self.decoder = Decoder(**config["Decoder"])
+        self.sn = bool(config["Decoder"].get("sn", False))
+        self._sn_dev: Dict[str, dict] = {}
         self._engines: Dict[str, Engine] = {}
         self._names_by_prefix = {}
         self._flat: Optional[torch.Tensor] = None
@@ -237,6 +252,84 @@ class AE(nn.Module):
             off += n
         self._flat = flat
         return flat
+
+    # ---- spectral normalisation of the decoder (sn: True)
+    def sn_layers(self) -> List[str]:
+        """The spectral-normalised layers ("decoder.in_conv_layer", ...) in registration order; [] without sn."""
+        if not self.sn:
+            return []
+        return [n[:-len(".weight_orig")] for n, _ in self.named_parameters() if n.endswith(".weight_orig")]
+
+    def _sn_state(self, device) -> dict:
+        """Per device: one buffer holding every layer's effective weight W/sigma and the sigma vector.  Allocated once
+        and never moved -- CUDA graphs and the engine's weight-pack tables hold their addresses."""
+        key = str(torch.device(device))
+        st = self._sn_dev.get(key)
+        if st is None:
+            params = dict(self.named_parameters())
+            layers = self.sn_layers()
+            shapes = [params[n + ".weight_orig"].shape for n in layers]
+            w = torch.zeros(sum(s.numel() for s in shapes), dtype=torch.float32, device=device)
+            views, off = {}, 0
+            for n, shp in zip(layers, shapes):
+                views[n] = w[off:off + shp.numel()].view(shp)
+                off += shp.numel()
+            st = self._sn_dev[key] = dict(w_sn=w, views=views, sigma=torch.zeros(len(layers), dtype=torch.float32, device=device),
+                                          tables={})
+        return st
+
+    def sn_views(self, P: Dict[str, torch.Tensor], G: Optional[Dict[str, torch.Tensor]] = None):
+        """The engine's view of the decoder's parameters: ``P["decoder.X.weight"]`` is the effective weight W/sigma
+        and ``G["decoder.X.weight"]`` aliases the gradient slot of ``decoder.X.weight_orig``.  The kernels then
+        write dL/d(W/sigma) there, which ``spectral_norm_bwd`` turns into dL/dweight_orig in place.  The other
+        entries are passed through; returns new dicts (P, G)."""
+        layers = self.sn_layers()
+        st = self._sn_state(P[layers[0] + ".weight_orig"].device)
+        P = dict(P, **{n + ".weight": st["views"][n] for n in layers})
+        if G is not None:
+            G = dict(G, **{n + ".weight": G[n + ".weight_orig"] for n in layers})
+        return P, G
+
+    def sigma(self, device) -> torch.Tensor:
+        """The 26 sigmas of the last spectral-norm forward on `device` (sn_layers() order)."""
+        return self._sn_state(device)["sigma"]
+
+    def sn_table(self, device, G=None) -> torch.Tensor:
+        """Device item table of avc_spectral_norm_fwd / _bwd (the gradient slots of G for the backward), cached
+        until an address changes.  Building it is a host-to-device copy: a CUDA-graph capture needs it built
+        before (FusedTrainer.capture does; Inferencer runs an eager call first)."""
+        st = self._sn_state(device)
+        params, bufs = dict(self.named_parameters()), dict(self.named_buffers())
+        layers = self.sn_layers()
+        rows = []
+        for i, n in enumerate(layers):
+            w = params[n + ".weight_orig"]
+            rows.append((w.data_ptr(), st["views"][n].data_ptr(), bufs[n + ".weight_u"].data_ptr(), bufs[n + ".weight_v"].data_ptr(),
+                         st["sigma"].data_ptr() + 4 * i, 0 if G is None else G[n + ".weight"].data_ptr(),
+                         w.shape[0], w.numel() // w.shape[0]))
+        key = tuple(rows)
+        hit = st["tables"].get(G is None)
+        if hit is None or hit[0] != key:
+            items = (L.SnItem * len(rows))()
+            for it, r in zip(items, rows):
+                it.w_orig, it.w_sn, it.u, it.v, it.sigma, it.grad, it.rows, it.cols = r
+            hit = st["tables"][G is None] = (key, torch.frombuffer(bytearray(bytes(items)), dtype=torch.uint8).to(device))
+        return hit[1]
+
+    def spectral_norm_fwd(self, device, update: bool):
+        """W/sigma of every decoder layer into the effective-weight buffer (one launch).  update (module.training in
+        the reference): one power iteration first, u and v overwritten; otherwise sigma from the stored u, v."""
+        lib = L.load()
+        st = torch.cuda.current_stream(device).cuda_stream
+        L.check(lib.avc_spectral_norm_fwd(self.sn_table(device).data_ptr(), len(self.sn_layers()), int(bool(update)), st),
+                "spectral_norm_fwd")
+
+    def spectral_norm_bwd(self, G):
+        """dL/d(W/sigma) -> dL/dweight_orig in place in G's slots (G as mapped by sn_views; one launch)."""
+        lib = L.load()
+        device = G[self.sn_layers()[0] + ".weight"].device
+        st = torch.cuda.current_stream(device).cuda_stream
+        L.check(lib.avc_spectral_norm_bwd(self.sn_table(device, G).data_ptr(), len(self.sn_layers()), st), "spectral_norm_bwd")
 
     # ---- the reference API
     def forward(self, x: torch.Tensor, *, eps: Optional[torch.Tensor] = None):

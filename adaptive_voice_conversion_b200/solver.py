@@ -98,9 +98,9 @@ class Solver(object):
     # ---- model + optimizer (solver.py:70-79)
     def build_model(self):
         self.model = cc(AE(self.config))
-        if self.world > 1:  # replicas start identical: broadcast rank 0's init
-            for p in self.model.parameters():
-                torch.distributed.broadcast(p.data, src=0)
+        if self.world > 1:  # replicas start identical: broadcast rank 0's init (and the spectral-norm u, v buffers)
+            for t in list(self.model.parameters()) + list(self.model.buffers()):
+                torch.distributed.broadcast(t.data, src=0)
         self.model.flatten_parameters()
         o = self.config["optimizer"]
         self.opt = FusedAdam(self.model, lr=o["lr"], betas=(o["beta1"], o["beta2"]), amsgrad=o["amsgrad"],

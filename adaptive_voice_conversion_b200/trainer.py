@@ -37,6 +37,8 @@ class FusedTrainer:
         self.lib = L.load()
         self.P: Dict[str, torch.Tensor] = dict(model.named_parameters())
         self.G: Dict[str, torch.Tensor] = opt.named_grad_views(model)
+        if model.sn:   # the kernels read W/sigma and write its gradient into the weight_orig slots (model.AE.sn_views)
+            self.P, self.G = model.sn_views(self.P, self.G)
         self.pg = process_group
         self.world = opt.world_size
         # one 16-byte report block so that reading a step's scalars is ONE device->host copy:
@@ -48,6 +50,7 @@ class FusedTrainer:
         self.n_rec = 1
         self.n_lat = 1
         self._graphs = None
+        self._graph_training = None   # the model.training a captured graph was recorded for (the power iteration runs only in training)
         self._static = None
         # the third consecutive step on the same batch shape (no injected eps) is recorded into CUDA graphs and every
         # later one replays them: a plain `Solver.train` loop gets the graph path without calling capture() (AVC_GRAPH=0: eager)
@@ -81,6 +84,12 @@ class FusedTrainer:
         eng, P, G = self.eng, self.P, self.G
         main, side = torch.cuda.current_stream(self.dev), self._side
         self.opt.zero_grad()
+        if self.model.sn:
+            # W/sigma (+ the power iteration in training mode) before any decoder kernel, then the step's one re-pack of
+            # the whole model (with sn it moves here from the end of the previous step, _update: a separate decoder
+            # pack would bump the pack version and make the lazily packed stride-2 encoder layers re-pack every step)
+            self.model.spectral_norm_fwd(self.dev, update=self.model.training)
+            eng.pack_weights(P, need_dgrad=True)
         # ---- forward: speaker branch || content branch (both only read x), joined in front of the decoder
         if side is not None:
             side.wait_stream(main)
@@ -138,6 +147,8 @@ class FusedTrainer:
         eng.wgrad_stream = self._wgs
         eng.join_wgrad()    # the forked weight gradients (of both branches) before their accumulators are flushed
         eng.flush_wgrad()   # no-op unless weight gradients were accumulated in place (AVC_WGRAD_ACC=1)
+        if self.model.sn:   # every decoder weight gradient is final here (flushes and both streams joined)
+            self.model.spectral_norm_bwd(G)
         return mu, ls, emb, dec
 
     def _allreduce(self):
@@ -146,7 +157,8 @@ class FusedTrainer:
 
     def _update(self):
         self.opt.step()
-        self.eng.pack_weights(self.P, need_dgrad=True)
+        if not self.model.sn:    # with sn the next step packs, from W/sigma (_fwd_bwd)
+            self.eng.pack_weights(self.P, need_dgrad=True)
 
     def set_lambda_kl(self, lambda_kl: float):
         """Push lambda_kl and the optimizer's param_group hyper-parameters (an lr scheduler may have changed
@@ -166,6 +178,8 @@ class FusedTrainer:
             raise L.AvcError("FusedTrainer.step: x must be a float32 CUDA tensor")
         x = x.contiguous()
         self.set_lambda_kl(lambda_kl)
+        if self._graphs is not None and self._graph_training != self.model.training:
+            self._graphs = None      # recorded for the other mode: record again
         replay = self._graphs is not None and tuple(x.shape) == tuple(self._static.shape) and not return_outputs
         if replay and (eps is None) == (self._static_eps is None):
             if x.data_ptr() != self._static.data_ptr():
@@ -205,12 +219,16 @@ class FusedTrainer:
         lam = self._lambda_kl if self._lambda_kl is not None else float(self.cfg["lambda"]["lambda_kl"])
         self.eng.prepare_tables(self.P, self.G)
         self.eng.prepare_wgrad_acc(self.P, self.G)
+        if self.model.sn:    # the spectral-norm item tables as well (host-to-device copies)
+            self.model.sn_table(self.dev)
+            self.model.sn_table(self.dev, self.G)
         self._graphs = None
         self._static = x_example.contiguous().clone()
         self._static_eps = None if eps_example is None else eps_example.contiguous().clone()
         for _ in range(warmup):
             self.step(self._static, lam, eps=self._static_eps)
         torch.cuda.synchronize(self.dev)
+        self._graph_training = self.model.training
         ga = torch.cuda.CUDAGraph()
         pool = torch.cuda.graph_pool_handle()
         if self.world == 1:    # one process: the whole step (zero-grad .. weight re-pack) is ONE graph

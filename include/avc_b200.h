@@ -329,6 +329,29 @@ int avc_adam_step(float* p, const float* g, float* m, float* v, float* vmax, int
 
 int avc_fill_zero(void* ptr, int64_t bytes, void* stream);
 
+/* Spectral normalisation of the decoder layers (torch.nn.utils.spectral_norm, dim=0, one power
+ * iteration, eps=1e-12; model.py:334-344 with sn: True).  One item per layer, Wm = w_orig viewed as
+ * [rows][cols] (rows = Cout, cols = Cin*K or in_features).  Both calls take a DEVICE-resident item
+ * table and run one CTA per item; every reduction has a fixed order (no atomics), so u, v, sigma and
+ * the outputs are bit-identical run to run.
+ * avc_spectral_norm_fwd, update != 0 (module.training): v = normalize(Wm^T u), u = normalize(Wm v)
+ *   (normalize(x) = x / max(|x|, 1e-12)), written back to u / v; then sigma = u . (Wm v) and
+ *   w_sn = w_orig / sigma.  update == 0: sigma from the stored u, v; u and v are not written.  grad is
+ *   not read.
+ * avc_spectral_norm_bwd: grad holds dL/dw_sn on entry and dL/dw_orig on return (u, v constants):
+ *   grad = (grad - <grad, w_sn> u v^T) / sigma, with the sigma / w_sn of the last forward. */
+typedef struct avc_sn_item {
+  const float* w_orig; /* [rows][cols] */
+  float* w_sn;         /* [rows][cols] w_orig / sigma */
+  float* u;            /* [rows] */
+  float* v;            /* [cols] */
+  float* sigma;        /* [1] */
+  float* grad;         /* [rows][cols], backward only (may be null for the forward) */
+  int32_t rows, cols;
+} avc_sn_item;
+int avc_spectral_norm_fwd(const avc_sn_item* items_dev, int n_items, int update, void* stream);
+int avc_spectral_norm_bwd(const avc_sn_item* items_dev, int n_items, void* stream);
+
 /* tcgen05 self-test (one CTA): D[128][N] = sum_k A_k * B_k^T over nk K=8 tf32 steps, the
  * operands given as raw shared-memory images; strides[10] = {a_lbo, a_sbo, b_lbo, b_sbo,
  * a_kstep, b_kstep, a_off, b_off (bytes), a_layout, b_layout (UMMA swizzle code, 0 = none)}; a_mn/b_mn = 1 for MN-major operands; the nk steps
